@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py ... --dump-outputs DIR      also writes the last timed step's seal and roots as DIR/seal.npy, DIR/roots.npy
 
 A "step" proves ONE synthetic 2^20-cycle segment of the SYN-280 circuit (BASELINE.json configs[1]; SURVEY.md 8d):
 iNTT + zk-shift, x4 coset LDE, Poseidon2 row hashing + Merkle commit for the code/data/accum/check groups,
@@ -35,6 +36,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 
 ORIG_AFFINITY = os.sched_getaffinity(0) if hasattr(os, "sched_getaffinity") else None
 METRIC = "segments proven/sec (2^20 cycles)"
@@ -130,15 +132,24 @@ def cpu_baseline(sample_po2, threads=None):
     pr.begin(sample_po2, io, code, data)
     pr.finish(accum)
     dt = time.time() - t0
-    return dt, cores
+    return dt, cores, pr
+
+
+def dump_outputs(out_dir, arrays, rank=0):
+    """--dump-outputs: every array as <out_dir>/<name>.npy in float64 (exact for u32 words), so that two builds can be compared
+    output for output; ranks other than 0 add _rank<r> to the name."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + (f"_rank{rank}" if rank else "") + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def reference_arm(args):
     """--impl reference: the reference's CPU implementation of the path.  The Rust crates cannot be built here (no
     cargo, source un-vendored), so this is the oracle port (oracle/, C++/OpenMP restatement of CpuHal) on all host threads.
     Every timed step proves one REAL SYN-280 segment of 2^20 cycles (no extrapolation): `value` = segments / measured seconds.
-    A full segment takes 20-40 s on a GPU box's host cores, so the number of timed steps is capped by a wall-clock budget
-    (--ref-budget-s, default 150 s; at least one step): `steps` is what was timed, `steps_requested` what the command line asked."""
+    A full segment takes 20-40 s on 16 host cores, so --ref-budget-s S can cap the timed steps at a wall-clock budget (at least
+    one step): `steps` is what was timed, `steps_requested` what the command line asked.  Without it every requested step runs."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -148,10 +159,10 @@ def reference_arm(args):
         warm.append(cpu_baseline(min(po2, 14))[0])             # untimed: loads the library, spins up the OpenMP team
     times, cores = [], 0
     t_start = time.time()
-    while len(times) < max(1, args.steps):
-        dt, cores = cpu_baseline(po2)
+    while len(times) < args.steps:
+        dt, cores, pr = cpu_baseline(po2)
         times.append(dt)
-        if (time.time() - t_start) + dt > args.ref_budget_s:      # the next step would not fit
+        if args.ref_budget_s is not None and (time.time() - t_start) + dt > args.ref_budget_s:      # the next step would not fit
             break
     ms = 1000.0 * sum(times) / len(times)
     value = 1000.0 / ms
@@ -164,6 +175,8 @@ def reference_arm(args):
             "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "port", "sample": sample},
             "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0,
             "steps_capped_by": None if len(times) >= args.steps else f"--ref-budget-s {args.ref_budget_s:.0f} (a full CPU segment proof takes {ms / 1000:.0f} s)"}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"seal": pr.seal(), "roots": pr.roots()})
     print(json.dumps(line), flush=True)
 
 
@@ -184,7 +197,7 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--po2", type=int, default=PO2, help="debug only: any value other than 20 is not the benchmark config")
     ap.add_argument("--cpu-sample-po2", type=int, default=0, help="cpu_baseline leg of the GPU arm: prove a 2^k-cycle segment instead of the full 2^20 one (debug)")
-    ap.add_argument("--ref-budget-s", type=float, default=150.0, help="--impl reference: wall-clock budget for the timed full-size CPU segment proofs (at least one is run)")
+    ap.add_argument("--ref-budget-s", type=float, default=None, help="--impl reference: wall-clock budget that may cut the timed full-size CPU segment proofs short of --steps (at least one is run)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--inflight", type=int, default=3, help="segments proven concurrently per GPU (one host thread + stream each)")
     ap.add_argument("--breakdown", action="store_true", help="per-operator timings to stderr")
@@ -192,7 +205,10 @@ def main():
                     help="syn280 = the benchmark segment (BASELINE configs[1]); synheavy = the SAME segment shape with the rv32im-shaped SYN-HEAVY "
                          "constraint system (22 k constraints, 117 k steps): a SECONDARY, eval_check-weighted line, not the headline")
     ap.add_argument("--session-segments", type=int, default=64, help="segments of the synthetic TLS session timed for the 'e2e TLS prove s' metric (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the seal and roots of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         reference_arm(args)
         return
@@ -356,6 +372,7 @@ def main():
     barrier()
     t1 = time.time()
     wall = t1 - t0
+    roots = prover.roots()          # worker 0 proves the first timed segment, and `seal` is its last one
     launches = sum(h.kernel_launches() for h in hals) - l0
     clocks = sampler.stop(t0, t1)
     t = torch.tensor([ms_dev], device=dev, dtype=torch.float64)
@@ -514,7 +531,7 @@ def main():
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline and not heavy:
         sample_po2 = args.cpu_sample_po2 or po2
-        dt, cores = cpu_baseline(sample_po2)
+        dt, cores, _ = cpu_baseline(sample_po2)
         scale = 1 << (po2 - sample_po2)
         cpu = {"value": 1.0 / (dt * scale), "unit": UNIT, "cores": cores, "kind": "port",
                "sample": f"oracle prover (C++/OpenMP restatement of CpuHal) on one SYN-280 segment of 2^{sample_po2} cycles: {dt:.2f} s"
@@ -555,6 +572,8 @@ def main():
                                          "constraint system (rv32im-shaped: 22 k constraints / 117 k PolyExtSteps, AndCond depth 4, taps back 0..4, 5 combos) -- eval_check-weighted companion of the headline"
             line["eval_check"] = ec
         print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"seal": seal, "roots": roots}, rank)
     for pr in provers:
         pr.close()
     if world > 1:
