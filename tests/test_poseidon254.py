@@ -31,8 +31,9 @@ def test_product_host_permutation_reproduces_the_known_answers_and_the_oracle():
     for _ in range(5):
         vals = [int.from_bytes(rng.bytes(32), "little") % O254.P for _ in range(3)]
         assert _host_permute(vals) == O254.permute(vals)
-    # edge values: 0, p - 1, and a 256-bit word above p (reduced on input)
+    # edge values: 0, p - 1, and a 256-bit word above p (reduced on input: 2^256 - 1 takes five subtractions of p)
     assert _host_permute([0, O254.P - 1, 1]) == O254.permute([0, O254.P - 1, 1])
+    assert _host_permute([0, (1 << 256) - 1, 1]) == O254.permute([0, ((1 << 256) - 1) % O254.P, 1])
 
 
 @pytest.fixture(scope="module")

@@ -1388,7 +1388,9 @@ bool eval_check_jit(zkb_ctx* ctx, uint32_t* d_check, const CircuitDef& c, const 
   bool aligned = ((uintptr_t)d_check & 15) == 0;
   for (int g = 0; g < 3; ++g) if ((uintptr_t)d_groups[g] & 15) aligned = false;
   const EvalJitKernel* k = nullptr;
-  if (flat_wanted(c) && aligned) {      // heavy circuit: flat form or nothing (the interpreter is the fallback, not a ten-minute compile)
+  if (flat_wanted(c)) {      // heavy circuit: flat form or nothing (the interpreter is the fallback, not a ten-minute compile)
+    // the flat / compact forms stage columns with 16-byte copies; an unaligned sub-buffer view goes to the interpreter
+    if (!aligned) { why = "heavy circuit on a buffer that is not 16-byte aligned"; return false; }
     k = get_kernel(ctx, c, false, why, true);
     if (k && domain < (size_t)k->points) { why = "domain smaller than one flat tile"; return false; }
     if (!k) return false;
