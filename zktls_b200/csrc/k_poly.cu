@@ -460,6 +460,19 @@ __global__ void k_pp_serial(uint4* __restrict__ io, size_t n) {
   }
 }
 
+// ---- exact comparison: *differ = 1 if any element differs (V = uint4 when both arrays are 16-byte aligned) ----------------
+__device__ __forceinline__ uint32_t bits_xor(uint32_t x, uint32_t y) { return x ^ y; }
+__device__ __forceinline__ uint32_t bits_xor(const uint4& x, const uint4& y) { return (x.x ^ y.x) | (x.y ^ y.y) | (x.z ^ y.z) | (x.w ^ y.w); }
+template <typename V>
+__global__ void __launch_bounds__(EW_BLOCK) k_differ(const V* __restrict__ a, const V* __restrict__ b, size_t count,
+                                                     const uint32_t* __restrict__ a_tail, const uint32_t* __restrict__ b_tail, uint32_t tail,
+                                                     uint32_t* __restrict__ differ) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  uint32_t d = i < count ? bits_xor(a[i], b[i]) : 0u;
+  if (i < tail) d |= a_tail[i] ^ b_tail[i];
+  if (__syncthreads_or(d != 0) && threadIdx.x == 0) *differ = 1u;
+}
+
 // ---- host-side launchers (shared with prover.cu) --------------------------------------------------------
 void eltwise_add(zkb_ctx* ctx, uint32_t* o, const uint32_t* a, const uint32_t* b, size_t n) {
   if (!n) return;
@@ -590,6 +603,25 @@ void prefix_products(zkb_ctx* ctx, uint32_t* d_io, size_t n) {
   prefix_products(ctx, (uint32_t*)totals, chunks);
   k_pp_apply<<<grid_for(chunks, 128), 128, 0, ctx->stream>>>((uint4*)d_io, totals, n); launched(ctx);
   pool_free(ctx, totals);
+}
+bool words_equal(zkb_ctx* ctx, const uint32_t* a, const uint32_t* b, size_t n) {
+  if (!n) return true;
+  uint32_t* flag = nullptr;
+  pool_alloc(ctx, &flag, 4);
+  ZKB_CUDA(cudaMemsetAsync(flag, 0, 4, ctx->stream));
+  if (aligned16(a) && aligned16(b)) {
+    const size_t n4 = n / 4;
+    const uint32_t tail = (uint32_t)(n % 4);
+    k_differ<uint4><<<grid_for(std::max<size_t>(n4, tail), EW_BLOCK), EW_BLOCK, 0, ctx->stream>>>((const uint4*)a, (const uint4*)b, n4, a + 4 * n4, b + 4 * n4, tail, flag);
+  } else {
+    k_differ<uint32_t><<<grid_for(n, EW_BLOCK), EW_BLOCK, 0, ctx->stream>>>(a, b, n, a, b, 0, flag);
+  }
+  launched(ctx);
+  uint32_t differ = 1;
+  ZKB_CUDA(cudaMemcpyAsync(&differ, flag, 4, cudaMemcpyDeviceToHost, ctx->stream));
+  ZKB_CUDA(cudaStreamSynchronize(ctx->stream));
+  pool_free(ctx, flag);
+  return differ == 0;
 }
 
 }  // namespace zkb

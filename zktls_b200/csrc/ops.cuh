@@ -32,6 +32,8 @@ void batch_evaluate_any(zkb_ctx* ctx, const uint32_t* coeffs, int po2, const uin
                         bool coeffs_bit_reversed = false);
 void poly_divide(zkb_ctx* ctx, uint32_t* d_poly, size_t n, const Fp4& z, uint32_t* d_rem);
 void prefix_products(zkb_ctx* ctx, uint32_t* d_io, size_t n);
+// true if the n words at a and b are all equal: one device pass, one 4-byte read-back (synchronises the stream)
+bool words_equal(zkb_ctx* ctx, const uint32_t* a, const uint32_t* b, size_t n);
 // CircuitHal::accumulate: the circuit blob's witness program, phase by phase (k_accum.cu)
 void accumulate(zkb_ctx* ctx, const CircuitDef& c, uint32_t* d_accum, const uint32_t* d_code, const uint32_t* d_data, const uint32_t* h_mix, const uint32_t* h_io, int po2);
 // k_eval_check.cu

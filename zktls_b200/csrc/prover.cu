@@ -61,6 +61,7 @@ struct DeviceMerkle {
   const uint32_t* matrix = nullptr;   // cols x rows, not owned
   DevBuf nodes;                       // 2*rows digests
   Digest root;
+  std::vector<uint32_t> top;          // the top layer, nodes[top_size .. 2*top_size), as commit() read it back
   void build(zkb_ctx* ctx, const uint32_t* m, size_t rows, size_t cols) {
     params = MerkleParams(rows, cols, QUERIES);
     matrix = m;
@@ -70,10 +71,15 @@ struct DeviceMerkle {
   }
   // MerkleTreeProver::commit: write the top layer, then mix the root.  One small blocking copy.
   void commit(zkb_ctx* ctx, WriteIOP& iop) {
-    std::vector<uint32_t> top(2 * params.top_size * 8);
-    d2h(ctx, top.data() + 8, nodes.p + 8, (2 * params.top_size - 1) * 32);    // nodes[1 .. 2*top_size)
-    iop.write(top.data() + params.top_size * 8, params.top_size * 8);
-    memcpy(root.w, top.data() + 8, 32);
+    std::vector<uint32_t> upper(2 * params.top_size * 8);
+    d2h(ctx, upper.data() + 8, nodes.p + 8, (2 * params.top_size - 1) * 32);    // nodes[1 .. 2*top_size)
+    top.assign(upper.begin() + params.top_size * 8, upper.end());
+    memcpy(root.w, upper.data() + 8, 32);
+    write(iop);
+  }
+  // the transcript actions of commit() for a tree committed before: the same top layer and root, no device work
+  void write(WriteIOP& iop) const {
+    iop.write(top.data(), top.size());
     iop.commit(root);
   }
   QueryTree query_tree(uint32_t out_offset) const {
@@ -149,8 +155,17 @@ struct zkb_prover {
   CircuitDef circuit;
   std::unique_ptr<WriteIOP> iop;
   int po2 = 0; size_t n = 0;
-  PolyGroup groups[3];
+  PolyGroup groups[3];            // this segment's accum and data groups; the code group is code.group (see group())
   PolyGroup check_group;
+  // The code group is the program: zkb_verify_segment accepts a seal only if its code root is one of the circuit's control IDs for
+  // that po2, so every valid proof of a circuit at one po2 commits the same code trace.  The last code commit that completed is kept
+  // across segments (reset() leaves it alone) and reused when the next code trace is equal to it word for word (~640 MB at po2 20).
+  struct CodeCommit {
+    int po2 = -1;                 // -1: nothing retained
+    DevBuf trace;                 // private copy of the committed trace (cols x n): the caller's buffer may change under the same pointer
+    PolyGroup group;              // coefficients, LDE matrix, Merkle tree with its top layer and root
+  } code;
+  const PolyGroup& group(int g) const { return g == GROUP_CODE ? code.group : groups[g]; }
   std::vector<std::unique_ptr<FriRound>> fri_rounds;
   std::vector<Digest> roots;
   std::vector<uint32_t> io, mix;
@@ -248,6 +263,7 @@ struct zkb_prover {
     PhaseTimer pt(ctx);
     size_t cols = circuit.group_size[g];
     if (group_ready) ZKB_CUDA(cudaStreamWaitEvent(ctx->stream, group_ready[g], 0));
+    if (g == GROUP_CODE) { commit_code(trace, on_device, pt); return; }
     DevBuf c(ctx, cols * n);
     // a trace that is already on the device is read in place by the first iNTT pass (no device-to-device copy)
     if (cols && !on_device) ZKB_CUDA(cudaMemcpyAsync(c.p, trace, cols * n * 4, cudaMemcpyHostToDevice, ctx->stream));
@@ -259,6 +275,44 @@ struct zkb_prover {
     groups[g].merkle.commit(ctx, *iop);
     pt.mark("commit_group: commit (d2h)");
     roots.push_back(groups[g].merkle.root);
+  }
+
+  // The code group: with the trace in device memory, compare it with the retained one.  Equal: the commitment is reused and only its
+  // transcript actions are replayed.  Different, or another po2: commit as above, then retain the result.
+  void commit_code(const void* trace, bool on_device, PhaseTimer& pt) {
+    const size_t cols = circuit.group_size[GROUP_CODE], words = cols * n;
+    DevBuf up;
+    if (!on_device) {
+      up = DevBuf(ctx, words);
+      if (words) ZKB_CUDA(cudaMemcpyAsync(up.p, trace, words * 4, cudaMemcpyHostToDevice, ctx->stream));
+      trace = up.p;
+      pt.mark("commit_group: upload");
+    }
+    const uint32_t* t = (const uint32_t*)trace;
+    if (code.po2 == po2 && words_equal(ctx, t, code.trace.p, words)) {
+      code.group.merkle.write(*iop);
+      roots.push_back(code.group.merkle.root);
+      pt.mark("commit_group: code reused");
+      return;
+    }
+    code = CodeCommit();          // dropped before the commit: an error in it leaves nothing retained, not a half-updated state
+    CodeCommit next;
+    if (up.p) {
+      next.trace = std::move(up);
+    } else {
+      next.trace = DevBuf(ctx, words);
+      if (words) ZKB_CUDA(cudaMemcpyAsync(next.trace.p, t, words * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+    DevBuf c(ctx, words);
+    ntt_inverse(ctx, c.p, cols, po2, true, next.trace.p);      // out of place: the retained copy keeps the trace
+    pt.mark("commit_group: iNTT+zk_shift");
+    next.group.build(ctx, std::move(c), cols, po2);
+    pt.mark("commit_group: LDE+hash+merkle");
+    next.group.merkle.commit(ctx, *iop);
+    pt.mark("commit_group: commit (d2h)");
+    roots.push_back(next.group.merkle.root);
+    next.po2 = po2;
+    code = std::move(next);
   }
 
   void segment_begin(int po2_, const uint32_t* h_io, const void* code, const void* data, bool on_device, uint32_t* h_mix_out) {
@@ -298,7 +352,7 @@ struct zkb_prover {
     Fp4 poly_mix = io_p.rng.random_ext_elem();
     {
       DevBuf check(ctx, EXT_SIZE * domain);
-      const uint32_t* ev[3] = {groups[0].evaluated.p, groups[1].evaluated.p, groups[2].evaluated.p};
+      const uint32_t* ev[3] = {group(0).evaluated.p, group(1).evaluated.p, group(2).evaluated.p};
       eval_check(ctx, check.p, c, ev, mix.data(), io.data(), poly_mix, po2);
       pt.mark("finalize: eval_check");
       ntt_inverse(ctx, check.p, EXT_SIZE, po2 + 2, false);
@@ -322,7 +376,7 @@ struct zkb_prover {
       h2d(ctx, d_xs.p, all_xs.data(), all_xs.size() * 16);
       for (uint32_t g = 0; g < 3; ++g) {
         size_t b = c.group_tap_begin(g), e = c.group_tap_end(g);
-        batch_evaluate_any(ctx, groups[g].coeffs.p, po2, d_which.p + b, d_xs.p + 4 * b, d_out.p + 4 * b, e - b, true);
+        batch_evaluate_any(ctx, group(g).coeffs.p, po2, d_which.p + b, d_xs.p + 4 * b, d_out.p + 4 * b, e - b, true);
       }
       batch_evaluate_any(ctx, check_group.coeffs.p, po2, d_which.p + tap_size, d_xs.p + 4 * tap_size, d_out.p + 4 * tap_size, CHECK_SIZE, true);
       d2h(ctx, eval_u.data(), d_out.p, eval_u.size() * 16);
@@ -350,7 +404,7 @@ struct zkb_prover {
       size_t off = 0;
       for (uint32_t g = 0; g < 3; ++g) {
         size_t cols = c.group_size[g];
-        mix_poly_coeffs(ctx, combos.p, cur, mix_c, groups[g].coeffs.p, d_ids.p + off, cols, n, (uint32_t)combos_size + 1);
+        mix_poly_coeffs(ctx, combos.p, cur, mix_c, group(g).coeffs.p, d_ids.p + off, cols, n, (uint32_t)combos_size + 1);
         cur *= pow(mix_c, cols);
         off += cols;
       }
@@ -436,7 +490,7 @@ struct zkb_prover {
     }
     std::vector<QueryTree> trees;
     uint32_t off = 0;
-    const DeviceMerkle* gm[4] = {&groups[0].merkle, &groups[1].merkle, &groups[2].merkle, &check_group.merkle};
+    const DeviceMerkle* gm[4] = {&group(0).merkle, &group(1).merkle, &group(2).merkle, &check_group.merkle};
     for (int t = 0; t < 4; ++t) { trees.push_back(gm[t]->query_tree(off)); off += gm[t]->query_words(); }
     for (auto& r : fri_rounds) { trees.push_back(r->merkle.query_tree(off)); off += r->merkle.query_words(); }
     const uint32_t words_per_query = off;
@@ -491,7 +545,7 @@ zkb_err zkb_prover_new(zkb_ctx* ctx, const uint32_t* h_circuit, size_t circuit_w
 }
 zkb_err zkb_prover_free(zkb_prover* p) {
   ZKB_API_BEGIN
-  if (p) { use(p->ctx); p->reset(); cudaStreamSynchronize(p->ctx->stream); if (p->copy_stream) cudaStreamSynchronize(p->copy_stream); p->free_staging(); delete p; }
+  if (p) { use(p->ctx); p->reset(); p->code = zkb_prover::CodeCommit(); cudaStreamSynchronize(p->ctx->stream); if (p->copy_stream) cudaStreamSynchronize(p->copy_stream); p->free_staging(); delete p; }
   ZKB_API_END
 }
 zkb_err zkb_prover_segment_begin(zkb_prover* p, int po2, const uint32_t* h_io, const void* code, const void* data, int traces_on_device, uint32_t* h_mix_out) {
