@@ -32,6 +32,7 @@ extern "C" {
 
 typedef struct zkb_ctx zkb_ctx;
 typedef struct zkb_prover zkb_prover;
+typedef struct zkb_program zkb_program;
 typedef const char* zkb_err;
 
 /* ---- lifecycle -------------------------------------------------------------------------------------- */
@@ -158,7 +159,8 @@ zkb_err zkb_prover_free(zkb_prover* p);
 /* First half of prove_segment: transcript header, commit_group(code), commit_group(data), then draws the circuit's
  * `mix` globals (written to h_mix_out, mix_size words).  code/data: group_size x 2^po2 column-major trace
  * evaluations; `*_on_device` says whether the pointer is a device or a (preferably pinned) host pointer.  The
- * trace buffers are not modified. */
+ * trace buffers are not modified.  code == NULL with a program attached (zkb_prover_set_program): the program's
+ * commitment at po2 is the code group, as in zkb_prove_segment and zkb_prover_stage_traces. */
 zkb_err zkb_prover_segment_begin(zkb_prover* p, int po2, const uint32_t* h_io, const void* code, const void* data,
                                  int traces_on_device, uint32_t* h_mix_out);
 /* Second half: commit_group(accum), finalize (eval_check, DEEP, FRI, queries).  The seal is then available. */
@@ -183,6 +185,42 @@ zkb_err zkb_prove_staged(zkb_prover* p, const uint32_t* h_io);
  * one PCIe link take turns instead of splitting its bandwidth).  It only synchronises the prover's copy stream, so -- unlike
  * every other call on a prover -- it may run on another host thread while zkb_prove_staged is in progress. */
 zkb_err zkb_prover_stage_wait(zkb_prover* p);
+
+/* ---- Program: a circuit's code commitments, made once per device and po2 ------------------------------------------------------
+ * The code trace is the program: zkb_verify_segment accepts a seal only if (po2, code root) is one of the circuit's control IDs.
+ * A program commits the code trace once per po2 on the device and holds the commitment read-only (trace copy, coefficients,
+ * LDE matrix, Merkle tree: ~640 MB at po2 20, ~10 GB at po2 24); any number of provers on that device prove segments from it
+ * given only their data and accum traces.
+ *
+ * With a program attached, a NULL code argument to zkb_prover_segment_begin, zkb_prove_segment or zkb_prover_stage_traces means
+ * "the program's commitment at this po2".  The transcript is the one commit_group(code) writes (top layer written, root mixed,
+ * root recorded), so seal and roots equal those the same segment gives when its code trace is passed.  On the staged path with
+ * h_accum == NULL the witness program reads the program's copy of the code trace: only data (or data and accum) is uploaded.  A po2
+ * the program has not committed is an error string naming it, returned before the transcript is touched or any device work
+ * starts (in zkb_prover_stage_traces too); the prover stays usable.  A non-NULL code argument takes the trace path unchanged,
+ * including the prover's own retained code commitment, which a segment proven from the program neither reads nor changes.
+ *
+ * Sharing and lifetime.  Entries are immutable once zkb_program_commit returns: provers on other ctxs and streams of the device
+ * read them with no further synchronisation, and provers driven from different host threads may share one program (a commit of a
+ * new po2 may run while they prove from existing entries).  Ownership is shared: the caller's handle and every prover holding the
+ * program keep it alive, and its memory goes when the last of them lets go.  A prover lets go by detaching, by attaching another
+ * program, or by zkb_prover_free; it synchronises its stream first, so no read of the entries is outstanding.  The storage lives on
+ * a private stream and memory pool of the device, so it does not depend on the ctx passed to zkb_program_new. */
+/* ctx names the device only: the program does not keep the ctx, and it may outlive it. */
+zkb_err zkb_program_new(zkb_ctx* ctx, const uint32_t* h_circuit, size_t circuit_words, zkb_program** out);
+/* Commits the code trace at po2 on the device: iNTT + zk_shift, x4 LDE, hash_rows, Merkle build.  This is exactly what
+ * commit_group(code) computes.  Blocks until the commitment is complete.  Writes the control ID (po2, code root[8]) to
+ * h_control_id (9 words).  A po2 that is already committed is an error: entries are immutable.  code: code_cols x 2^po2 words,
+ * a device pointer (its contents complete before the call) when code_on_device, else a host pointer; it is not kept. */
+zkb_err zkb_program_commit(zkb_program* prog, int po2, const void* code, int code_on_device, uint32_t* h_control_id);
+/* The table zkb_verify_segment takes: *n entries of 9 words, ascending po2.  h_out == NULL only queries *n; otherwise *n is h_out's
+ * capacity in entries on input (an error if smaller than the table) and the number written on return. */
+zkb_err zkb_program_control_ids(zkb_program* prog, size_t* n, uint32_t* h_out);
+zkb_err zkb_program_free(zkb_program* prog);   /* releases the caller's handle; provers holding the program keep it alive */
+/* Attaches prog to p (NULL detaches).  The circuit blobs must be equal word for word, and both must be on the same device.
+ * A segment begun from the program keeps it alive until the prover's next segment or zkb_prover_free. */
+zkb_err zkb_prover_set_program(zkb_prover* p, zkb_program* prog);
+
 /* CPU verifier for a seal produced by the prover (risc0-zkp verify/*): checks the transcript, Merkle paths, FRI
  * and the constraint relation at the DEEP point.  Host-only, like the reference's verifier.
  * The code group's Merkle root identifies the PROGRAM (risc0: `check_code(po2, root)` against the control ID): it must equal

@@ -4,7 +4,7 @@ the output is source only; tests/test_abi_symbols.py checks that it is current a
 import os, re, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 TYPES = {"int": "c_int", "size_t": "usize", "uint32_t": "u32", "uint64_t": "u64", "float": "f32", "char": "c_char", "void": "c_void",
-         "zkb_ctx": "ZkbCtx", "zkb_prover": "ZkbProver"}
+         "zkb_ctx": "ZkbCtx", "zkb_prover": "ZkbProver", "zkb_program": "ZkbProgram"}
 
 
 def rust_type(ctype):
@@ -40,6 +40,7 @@ def generate():
              "//! Conventions are those of risc0-sys: every operator returns NULL or a malloc'd message (`ffi_wrap`).",
              "#![allow(non_camel_case_types)]", "use std::ffi::{c_char, c_int, c_void, CStr};", "",
              "#[repr(C)] pub struct ZkbCtx { _private: [u8; 0] }", "#[repr(C)] pub struct ZkbProver { _private: [u8; 0] }",
+             "#[repr(C)] pub struct ZkbProgram { _private: [u8; 0] }",
              "pub type ZkbErr = *const c_char;", "", '#[link(name = "zkb200")]', 'extern "C" {']
     for name, ret, params in fns:
         r = {"zkb_err": " -> ZkbErr", "const char*": " -> *const c_char", "void": ""}[ret]

@@ -29,6 +29,7 @@ SYMBOLS = [
     "zkb_prover_new", "zkb_prover_free", "zkb_prover_segment_begin", "zkb_prover_segment_finish", "zkb_prover_seal_words",
     "zkb_prover_seal_copy", "zkb_prover_root_count", "zkb_prover_roots_copy", "zkb_prove_segment", "zkb_prover_stage_traces",
     "zkb_prove_staged", "zkb_prover_stage_wait", "zkb_verify_segment",
+    "zkb_program_new", "zkb_program_commit", "zkb_program_control_ids", "zkb_program_free", "zkb_prover_set_program",
     "zkb_poseidon254_hash_rows", "zkb_poseidon254_hash_fold", "zkb_poseidon254_merkle_build", "zkb_poseidon254_permute_host",
 ]
 

@@ -71,11 +71,15 @@ struct DeviceMerkle {
   }
   // MerkleTreeProver::commit: write the top layer, then mix the root.  One small blocking copy.
   void commit(zkb_ctx* ctx, WriteIOP& iop) {
+    read_top(ctx);
+    write(iop);
+  }
+  // reads the top layer and the root back; blocks until the tree is built
+  void read_top(zkb_ctx* ctx) {
     std::vector<uint32_t> upper(2 * params.top_size * 8);
     d2h(ctx, upper.data() + 8, nodes.p + 8, (2 * params.top_size - 1) * 32);    // nodes[1 .. 2*top_size)
     top.assign(upper.begin() + params.top_size * 8, upper.end());
     memcpy(root.w, upper.data() + 8, 32);
-    write(iop);
   }
   // the transcript actions of commit() for a tree committed before: the same top layer and root, no device work
   void write(WriteIOP& iop) const {
@@ -123,7 +127,64 @@ struct PhaseTimer {
   }
 };
 
+// A completed commitment of the code group, i.e. of the program at one po2: a private copy of the trace (the witness program reads it,
+// and a caller's buffer may change under the same pointer), the bit-reversed coefficients, the LDE matrix and the Merkle tree with its
+// top layer and root (~640 MB at po2 20).  A prover keeps its last one (zkb_prover::code); a zkb_program keeps one per committed po2.
+struct CodeCommit {
+  int po2 = -1;                 // -1: empty
+  DevBuf trace;
+  PolyGroup group;
+  // Prover::commit_group(code) without its transcript actions (group.merkle.write replays those): make_coeffs out of place, so that
+  // the copy keeps the trace, PolyGroup::new, and the top-layer read-back.  `t` is the trace in device memory; `uploaded` is the buffer
+  // it was uploaded into, taken over as the copy, or empty when `t` is the caller's buffer and has to be copied.
+  void build(zkb_ctx* ctx, DevBuf&& uploaded, const uint32_t* t, size_t cols, int po2_, PhaseTimer& pt) {
+    const size_t words = cols << po2_;
+    if (uploaded.p) {
+      trace = std::move(uploaded);
+    } else {
+      trace = DevBuf(ctx, words);
+      if (words) ZKB_CUDA(cudaMemcpyAsync(trace.p, t, words * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+    DevBuf c(ctx, words);
+    ntt_inverse(ctx, c.p, cols, po2_, true, trace.p);
+    pt.mark("commit_group: iNTT+zk_shift");
+    group.build(ctx, std::move(c), cols, po2_);
+    pt.mark("commit_group: LDE+hash+merkle");
+    group.merkle.read_top(ctx);
+    pt.mark("commit_group: commit (d2h)");
+    po2 = po2_;
+  }
+};
+
+// zkb_program (include/zkb200.h): one circuit's code commitments, one per po2, built on a private ctx of the device (own stream and pool,
+// so the storage depends on no caller's ctx) and read by any prover on that device.  An entry is complete when zkb_program_commit returns
+// and is neither changed nor removed until the program is destroyed, so provers on other streams read it without synchronisation.
+// Ownership is shared between the caller's handle and every prover holding the program; each holder synchronises its stream before it
+// lets go (zkb_prover::release), so the last one frees memory no stream still reads.
+struct Program {
+  zkb_ctx* ctx = nullptr;
+  std::vector<uint32_t> blob;
+  CircuitDef circuit;
+  std::mutex commit_mu;                     // one commit at a time on the private ctx
+  mutable std::mutex map_mu;                // guards `entries` alone: provers look entries up while a new po2 is being committed
+  std::map<int, std::unique_ptr<CodeCommit>> entries;
+  const CodeCommit* find(int po2) const {
+    std::lock_guard<std::mutex> lock(map_mu);
+    auto it = entries.find(po2);
+    return it == entries.end() ? nullptr : it->second.get();
+  }
+  ~Program() {
+    if (!ctx) return;
+    cudaSetDevice(ctx->device);
+    entries.clear();                        // stream-ordered frees on the private stream
+    zkb_free_error(zkb_destroy(ctx));       // synchronises that stream, then destroys its pool
+  }
+};
+static std::string no_program_entry(int po2) { return "the attached program has no code commitment at po2 " + std::to_string(po2) + " (zkb_program_commit)"; }
+
 }  // namespace zkb
+
+struct zkb_program { std::shared_ptr<zkb::Program> s; };
 
 using namespace zkb;
 
@@ -152,20 +213,27 @@ static Digest hash_protocol_info(const uint8_t* info) {
 
 struct zkb_prover {
   zkb_ctx* ctx = nullptr;
+  std::vector<uint32_t> blob;
   CircuitDef circuit;
   std::unique_ptr<WriteIOP> iop;
   int po2 = 0; size_t n = 0;
-  PolyGroup groups[3];            // this segment's accum and data groups; the code group is code.group (see group())
+  PolyGroup groups[3];            // this segment's accum and data groups; the code group is seg_code's or code's (see group())
   PolyGroup check_group;
   // The code group is the program: zkb_verify_segment accepts a seal only if its code root is one of the circuit's control IDs for
   // that po2, so every valid proof of a circuit at one po2 commits the same code trace.  The last code commit that completed is kept
   // across segments (reset() leaves it alone) and reused when the next code trace is equal to it word for word (~640 MB at po2 20).
-  struct CodeCommit {
-    int po2 = -1;                 // -1: nothing retained
-    DevBuf trace;                 // private copy of the committed trace (cols x n): the caller's buffer may change under the same pointer
-    PolyGroup group;              // coefficients, LDE matrix, Merkle tree with its top layer and root
-  } code;
-  const PolyGroup& group(int g) const { return g == GROUP_CODE ? code.group : groups[g]; }
+  CodeCommit code;
+  // zkb_prover_set_program: a NULL code argument proves from the attached program's commitment at the segment's po2.  The segment
+  // holds the program it read from until reset(), so detaching mid-segment does not free what its finish still reads.
+  std::shared_ptr<Program> program, seg_program;
+  const CodeCommit* seg_code = nullptr;
+  const PolyGroup& group(int g) const { return g != GROUP_CODE ? groups[g] : seg_code ? seg_code->group : code.group; }
+  // lets go of a program: every read of its entries on this prover's stream must be done first
+  void release(std::shared_ptr<Program>& h) {
+    if (!h) return;
+    ZKB_CUDA(cudaStreamSynchronize(ctx->stream));
+    h.reset();
+  }
   std::vector<std::unique_ptr<FriRound>> fri_rounds;
   std::vector<Digest> roots;
   std::vector<uint32_t> io, mix;
@@ -181,6 +249,7 @@ struct zkb_prover {
     int po2 = -1;
     bool full = false;
     bool device_accum = false;      // no accum trace was staged: zkb_prove_staged fills the group with the circuit's witness program
+    bool code_from_program = false; // no code trace was staged: the attached program's commitment is used, and nothing is uploaded for it
   };
   TraceSlot slots[2];
   cudaStream_t copy_stream = nullptr;
@@ -190,6 +259,8 @@ struct zkb_prover {
 
   void stage_traces(int po2_, const void* const h_traces[3]) {
     ZKB_REQUIRE(po2_ >= 6 && po2_ + 2 <= MAX_PO2, "segment po2 out of range [6, 24]");
+    const bool code_from_program = !h_traces[GROUP_CODE] && program;
+    ZKB_REQUIRE(!code_from_program || program->find(po2_), no_program_entry(po2_));
     if (!copy_stream) {
       static const bool priv = [] { const char* e = getenv("ZKB_COPY_STREAM"); return e && !strcmp(e, "private"); }();      // measurement knob: one stream per prover (round-1 behaviour)
       if (priv) { ZKB_CUDA(cudaStreamCreateWithFlags(&copy_stream, cudaStreamNonBlocking)); own_copy_stream = true; }
@@ -210,7 +281,7 @@ struct zkb_prover {
     for (int k = 0; k < 3; ++k) {
       const int g = ORDER[k];
       size_t words = (size_t)circuit.group_size[g] * rows;
-      if (sl.words[g] < words) {
+      if (sl.words[g] < words && !(g == GROUP_CODE && code_from_program)) {
         if (sl.buf[g]) { ZKB_CUDA(cudaStreamSynchronize(ctx->stream)); ZKB_CUDA(cudaStreamSynchronize(copy_stream)); ZKB_CUDA(cudaFree(sl.buf[g])); }
         ZKB_CUDA(cudaMalloc((void**)&sl.buf[g], std::max<size_t>(words, 4) * 4));
         sl.words[g] = words;
@@ -219,6 +290,7 @@ struct zkb_prover {
       ZKB_CUDA(cudaEventRecord(sl.uploaded[g], copy_stream));
     }
     sl.device_accum = h_traces[GROUP_ACCUM] == nullptr && circuit.group_size[GROUP_ACCUM] != 0;
+    sl.code_from_program = code_from_program;
     sl.po2 = po2_; sl.full = true;
     stage_idx ^= 1;
   }
@@ -227,12 +299,13 @@ struct zkb_prover {
     ZKB_REQUIRE(sl.full, "no staged traces: call zkb_prover_stage_traces first");
     struct Guard { const cudaEvent_t*& r; ~Guard() { r = nullptr; } } guard{group_ready};      // also on an error path
     group_ready = sl.uploaded;
-    segment_begin(sl.po2, h_io, sl.buf[GROUP_CODE], sl.buf[GROUP_DATA], true, nullptr);
+    segment_begin(sl.po2, h_io, sl.code_from_program ? nullptr : sl.buf[GROUP_CODE], sl.buf[GROUP_DATA], true, nullptr);
     if (sl.device_accum) {
       // the reference's prove_segment order: commit code + data, draw `mix`, CircuitHal::accumulate, commit accum -- with the witness
       // program of the circuit blob run on the device, so this group (14 % of SYN-280's trace bytes) never crosses the host link
       ZKB_CUDA(cudaMemsetAsync(sl.buf[GROUP_ACCUM], 0, sl.words[GROUP_ACCUM] * 4, ctx->stream));
-      accumulate(ctx, circuit, sl.buf[GROUP_ACCUM], sl.buf[GROUP_CODE], sl.buf[GROUP_DATA], mix.data(), io.data(), sl.po2);
+      const uint32_t* code_trace = seg_code ? seg_code->trace.p : sl.buf[GROUP_CODE];      // the program's retained copy
+      accumulate(ctx, circuit, sl.buf[GROUP_ACCUM], code_trace, sl.buf[GROUP_DATA], mix.data(), io.data(), sl.po2);
     }
     segment_finish(sl.buf[GROUP_ACCUM], true);
     ZKB_CUDA(cudaEventRecord(sl.consumed, ctx->stream));
@@ -256,6 +329,8 @@ struct zkb_prover {
     check_group = PolyGroup();
     fri_rounds.clear(); roots.clear(); io.clear(); mix.clear();
     begun = finished = false;
+    seg_code = nullptr;
+    release(seg_program);
   }
 
   // Prover::commit_group: make_coeffs (interpolate + zk_shift), PolyGroup::new, merkle.commit
@@ -277,9 +352,16 @@ struct zkb_prover {
     roots.push_back(groups[g].merkle.root);
   }
 
-  // The code group: with the trace in device memory, compare it with the retained one.  Equal: the commitment is reused and only its
-  // transcript actions are replayed.  Different, or another po2: commit as above, then retain the result.
+  // The code group.  From the program: replay the transcript actions of its commitment; the prover's own retained commitment is
+  // neither read nor changed.  From a trace: with the trace in device memory, compare it with the retained one.  Equal: the commitment
+  // is reused and only its transcript actions are replayed.  Different, or another po2: commit, then retain the result.
   void commit_code(const void* trace, bool on_device, PhaseTimer& pt) {
+    if (seg_code) {
+      seg_code->group.merkle.write(*iop);
+      roots.push_back(seg_code->group.merkle.root);
+      pt.mark("commit_group: code from program");
+      return;
+    }
     const size_t cols = circuit.group_size[GROUP_CODE], words = cols * n;
     DevBuf up;
     if (!on_device) {
@@ -297,27 +379,23 @@ struct zkb_prover {
     }
     code = CodeCommit();          // dropped before the commit: an error in it leaves nothing retained, not a half-updated state
     CodeCommit next;
-    if (up.p) {
-      next.trace = std::move(up);
-    } else {
-      next.trace = DevBuf(ctx, words);
-      if (words) ZKB_CUDA(cudaMemcpyAsync(next.trace.p, t, words * 4, cudaMemcpyDeviceToDevice, ctx->stream));
-    }
-    DevBuf c(ctx, words);
-    ntt_inverse(ctx, c.p, cols, po2, true, next.trace.p);      // out of place: the retained copy keeps the trace
-    pt.mark("commit_group: iNTT+zk_shift");
-    next.group.build(ctx, std::move(c), cols, po2);
-    pt.mark("commit_group: LDE+hash+merkle");
-    next.group.merkle.commit(ctx, *iop);
-    pt.mark("commit_group: commit (d2h)");
+    next.build(ctx, std::move(up), t, cols, po2, pt);
+    next.group.merkle.write(*iop);
     roots.push_back(next.group.merkle.root);
-    next.po2 = po2;
     code = std::move(next);
   }
 
+  // code == NULL with a program attached: the program's commitment at po2_ is this segment's code group
   void segment_begin(int po2_, const uint32_t* h_io, const void* code, const void* data, bool on_device, uint32_t* h_mix_out) {
     ZKB_REQUIRE(po2_ >= 6 && po2_ + 2 <= MAX_PO2, "segment po2 out of range [6, 24]");
+    const CodeCommit* from_program = nullptr;
+    if (!code && program) {
+      from_program = program->find(po2_);
+      ZKB_REQUIRE(from_program, no_program_entry(po2_));
+    }
+    ZKB_REQUIRE(code || from_program || circuit.group_size[GROUP_CODE] == 0, "null code trace and no program attached");
     reset();
+    if (from_program) { seg_program = program; seg_code = from_program; }
     po2 = po2_; n = (size_t)1 << po2;
     iop->commit(hash_protocol_info((const uint8_t*)PROOF_SYSTEM_INFO));
     iop->commit(hash_protocol_info(circuit.info));
@@ -539,20 +617,97 @@ zkb_err zkb_prover_new(zkb_ctx* ctx, const uint32_t* h_circuit, size_t circuit_w
   std::unique_ptr<zkb_prover> p(new zkb_prover());
   p->ctx = ctx;
   p->circuit = CircuitDef::parse(h_circuit, circuit_words);
+  p->blob.assign(h_circuit, h_circuit + circuit_words);
   p->reset();
   *out = p.release();
   ZKB_API_END
 }
 zkb_err zkb_prover_free(zkb_prover* p) {
   ZKB_API_BEGIN
-  if (p) { use(p->ctx); p->reset(); p->code = zkb_prover::CodeCommit(); cudaStreamSynchronize(p->ctx->stream); if (p->copy_stream) cudaStreamSynchronize(p->copy_stream); p->free_staging(); delete p; }
+  if (p) {
+    use(p->ctx); p->reset(); p->code = CodeCommit(); cudaStreamSynchronize(p->ctx->stream); if (p->copy_stream) cudaStreamSynchronize(p->copy_stream); p->free_staging();
+    p->program.reset();      // the stream is synchronised above
+    delete p;
+  }
+  ZKB_API_END
+}
+zkb_err zkb_prover_set_program(zkb_prover* p, zkb_program* prog) {
+  ZKB_API_BEGIN
+  ZKB_REQUIRE(p != nullptr, "null prover");
+  use(p->ctx);
+  std::shared_ptr<Program> next;
+  if (prog) {
+    next = prog->s;
+    ZKB_REQUIRE(next->ctx->device == p->ctx->device, "the program was made for another device than the prover's");
+    ZKB_REQUIRE(next->blob == p->blob, "the program was made for another circuit blob than the prover's");
+  }
+  p->release(p->program);
+  p->program = std::move(next);
+  ZKB_API_END
+}
+zkb_err zkb_program_new(zkb_ctx* ctx, const uint32_t* h_circuit, size_t circuit_words, zkb_program** out) {
+  ZKB_API_BEGIN
+  use(ctx);
+  ZKB_REQUIRE(out != nullptr, "null out pointer");
+  std::shared_ptr<Program> s = std::make_shared<Program>();
+  s->circuit = CircuitDef::parse(h_circuit, circuit_words);
+  s->blob.assign(h_circuit, h_circuit + circuit_words);
+  if (zkb_err e = zkb_init(ctx->device, &s->ctx)) { std::string m(e); zkb_free_error(e); throw Error(m); }
+  *out = new zkb_program{std::move(s)};
+  ZKB_API_END
+}
+zkb_err zkb_program_commit(zkb_program* prog, int po2, const void* code, int code_on_device, uint32_t* h_control_id) {
+  ZKB_API_BEGIN
+  ZKB_REQUIRE(prog != nullptr, "null program");
+  Program& g = *prog->s;
+  ZKB_REQUIRE(po2 >= 6 && po2 + 2 <= MAX_PO2, "segment po2 out of range [6, 24]");
+  const size_t cols = g.circuit.group_size[GROUP_CODE], words = cols << po2;
+  ZKB_REQUIRE((code || cols == 0) && h_control_id, "null argument");
+  std::lock_guard<std::mutex> lock(g.commit_mu);
+  ZKB_REQUIRE(!g.find(po2), "the program already holds a code commitment at po2 " + std::to_string(po2) + " (entries are immutable)");
+  use(g.ctx);
+  PhaseTimer pt(g.ctx);
+  DevBuf up;
+  if (!code_on_device) {
+    up = DevBuf(g.ctx, words);
+    if (words) ZKB_CUDA(cudaMemcpyAsync(up.p, code, words * 4, cudaMemcpyHostToDevice, g.ctx->stream));
+    pt.mark("commit_group: upload");
+  }
+  const uint32_t* t = code_on_device ? (const uint32_t*)code : up.p;
+  std::unique_ptr<CodeCommit> e(new CodeCommit());
+  e->build(g.ctx, std::move(up), t, cols, po2, pt);      // ends in a blocking read-back: the entry is complete on return
+  h_control_id[0] = (uint32_t)po2;
+  memcpy(h_control_id + 1, e->group.merkle.root.w, 32);
+  std::lock_guard<std::mutex> map_lock(g.map_mu);
+  g.entries[po2] = std::move(e);
+  ZKB_API_END
+}
+zkb_err zkb_program_control_ids(zkb_program* prog, size_t* n, uint32_t* h_out) {
+  ZKB_API_BEGIN
+  ZKB_REQUIRE(prog && n, "null argument");
+  const Program& g = *prog->s;
+  std::lock_guard<std::mutex> lock(g.map_mu);
+  if (h_out) {
+    ZKB_REQUIRE(*n >= g.entries.size(), "h_out holds " + std::to_string(*n) + " entries; the program has " + std::to_string(g.entries.size()));
+    for (const auto& kv : g.entries) {
+      *h_out++ = (uint32_t)kv.first;
+      memcpy(h_out, kv.second->group.merkle.root.w, 32);
+      h_out += 8;
+    }
+  }
+  *n = g.entries.size();
+  ZKB_API_END
+}
+zkb_err zkb_program_free(zkb_program* prog) {
+  ZKB_API_BEGIN
+  delete prog;
   ZKB_API_END
 }
 zkb_err zkb_prover_segment_begin(zkb_prover* p, int po2, const uint32_t* h_io, const void* code, const void* data, int traces_on_device, uint32_t* h_mix_out) {
   ZKB_API_BEGIN
   ZKB_REQUIRE(p != nullptr, "null prover");
   use(p->ctx);
-  ZKB_REQUIRE((h_io || p->circuit.out_size == 0) && (code || p->circuit.group_size[GROUP_CODE] == 0) && (data || p->circuit.group_size[GROUP_DATA] == 0), "null argument");
+  ZKB_REQUIRE((h_io || p->circuit.out_size == 0) && (code || p->program || p->circuit.group_size[GROUP_CODE] == 0) && (data || p->circuit.group_size[GROUP_DATA] == 0), "null argument");
   p->segment_begin(po2, h_io, code, data, traces_on_device != 0, h_mix_out);
   ZKB_API_END
 }
@@ -568,8 +723,8 @@ zkb_err zkb_prove_segment(zkb_prover* p, int po2, const uint32_t* h_io, const vo
   ZKB_API_BEGIN
   ZKB_REQUIRE(p != nullptr, "null prover");
   use(p->ctx);
-  ZKB_REQUIRE((h_io || p->circuit.out_size == 0) && (code || p->circuit.group_size[GROUP_CODE] == 0) && (data || p->circuit.group_size[GROUP_DATA] == 0) &&
-              (accum || p->circuit.group_size[GROUP_ACCUM] == 0), "null argument");
+  ZKB_REQUIRE((h_io || p->circuit.out_size == 0) && (code || p->program || p->circuit.group_size[GROUP_CODE] == 0) &&
+              (data || p->circuit.group_size[GROUP_DATA] == 0) && (accum || p->circuit.group_size[GROUP_ACCUM] == 0), "null argument");
   p->segment_begin(po2, h_io, code, data, traces_on_device != 0, nullptr);
   p->segment_finish(accum, traces_on_device != 0);
   ZKB_API_END
@@ -580,7 +735,7 @@ zkb_err zkb_prover_stage_traces(zkb_prover* p, int po2, const void* h_code, cons
   use(p->ctx);
   const void* tr[3];
   tr[GROUP_ACCUM] = h_accum; tr[GROUP_CODE] = h_code; tr[GROUP_DATA] = h_data;
-  for (int g = 0; g < 3; ++g) ZKB_REQUIRE(tr[g] || p->circuit.group_size[g] == 0 || (g == GROUP_ACCUM && !p->circuit.wsteps.empty()),
+  for (int g = 0; g < 3; ++g) ZKB_REQUIRE(tr[g] || p->circuit.group_size[g] == 0 || (g == GROUP_ACCUM && !p->circuit.wsteps.empty()) || (g == GROUP_CODE && p->program),
                                           g == GROUP_ACCUM ? "null accum trace and the circuit blob carries no witness program to compute it" : "null trace");
   p->stage_traces(po2, tr);
   ZKB_API_END
