@@ -221,6 +221,40 @@ zkb_err zkb_program_free(zkb_program* prog);   /* releases the caller's handle; 
  * A segment begun from the program keeps it alive until the prover's next segment or zkb_prover_free. */
 zkb_err zkb_prover_set_program(zkb_prover* p, zkb_program* prog);
 
+/* ---- Session: the continuation segments of one session, proven on every device of the process ------------------------------------
+ * A session owns `inflight` worker threads per device, each with its own ctx and staged prover, and one program per device.  The caller
+ * commits the code trace once per po2, submits (po2, io, data[, accum]) per segment and collects seals by ticket; no per-device code
+ * and no threads of its own.  One queue serves every device, so a session's tail is one segment, not one round.  A worker stages its
+ * next segment while it proves the current one (zkb_prover_stage_traces / zkb_prove_staged, code from the program).  Within a device,
+ * uploads enter the shared copy stream in the order their segments leave the queue, and a worker does not prefetch a second segment
+ * while the queue is non-empty and another worker of its device has nothing staged (DESIGN.md section 6).  Device memory per device:
+ * inflight x (segment working set + 2 staging slots without the code group) + the program.  submit, wait and commit may be called from
+ * any host thread, concurrently; zkb_session_free must be the last call on a session. */
+typedef struct zkb_session zkb_session;
+/* devices == NULL: every visible device.  inflight: provers per device (1..8).  Starts inflight worker threads per device; each
+ * creates its own ctx and prover on its own thread (a ctx is driven by one host thread).  On an error nothing stays running. */
+zkb_err zkb_session_new(const uint32_t* h_circuit, size_t circuit_words, const int* devices, size_t n_devices, int inflight,
+                        zkb_session** out);
+/* Commits the code trace (host pointer) at po2 on every device of the session, in parallel, and writes the control ID (9 words).
+ * The per-device roots must agree: a mismatch is an error.  A po2 already committed is an error. */
+zkb_err zkb_session_commit(zkb_session* s, int po2, const void* h_code, uint32_t* h_control_id);
+zkb_err zkb_session_control_ids(zkb_session* s, size_t* n, uint32_t* h_out);    /* same convention as zkb_program_control_ids */
+/* Queues one segment; returns at once with a ticket (increasing in submit order).  h_io is copied.  h_data / h_accum (pinned
+ * recommended; pageable works) must stay alive and unmodified until the ticket's seal has been collected or the session is freed.
+ * h_accum == NULL: the circuit's witness program computes the accum group on the device.  Refused here, with nothing queued,
+ * for: a po2 that has not been committed (named in the message), NULL data with data_cols > 0, NULL accum with no witness program
+ * in the blob, or a session being freed.  A segment that fails later (e.g. an io word >= P) fails its own ticket only. */
+zkb_err zkb_session_submit(zkb_session* s, int po2, const uint32_t* h_io, const void* h_data, const void* h_accum, uint64_t* ticket);
+/* Blocks until the ticket's segment is proven.  h_seal == NULL: writes the seal length to *words and keeps the result.
+ * Otherwise *words is h_seal's capacity on input (an error if smaller than the seal); copies the seal, sets *words, releases the
+ * ticket.  A segment that failed returns its own error string, once, and the ticket is released.  Unknown or released
+ * ticket: error. */
+zkb_err zkb_session_wait(zkb_session* s, uint64_t ticket, uint32_t* h_seal, size_t* words);
+/* Stops accepting segments.  Segments whose proof has not started (queued, or staged ahead on a worker) fail with "session freed".
+ * Waits for the proofs in progress and for the threads inside zkb_session_wait, joins every worker thread, then frees the provers,
+ * programs and ctxs. */
+zkb_err zkb_session_free(zkb_session* s);
+
 /* CPU verifier for a seal produced by the prover (risc0-zkp verify/*): checks the transcript, Merkle paths, FRI
  * and the constraint relation at the DEEP point.  Host-only, like the reference's verifier.
  * The code group's Merkle root identifies the PROGRAM (risc0: `check_code(po2, root)` against the control ID): it must equal

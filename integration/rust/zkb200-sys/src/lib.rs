@@ -6,6 +6,7 @@ use std::ffi::{c_char, c_int, c_void, CStr};
 #[repr(C)] pub struct ZkbCtx { _private: [u8; 0] }
 #[repr(C)] pub struct ZkbProver { _private: [u8; 0] }
 #[repr(C)] pub struct ZkbProgram { _private: [u8; 0] }
+#[repr(C)] pub struct ZkbSession { _private: [u8; 0] }
 pub type ZkbErr = *const c_char;
 
 #[link(name = "zkb200")]
@@ -74,6 +75,12 @@ extern "C" {
     pub fn zkb_program_control_ids(prog: *mut ZkbProgram, n: *mut usize, h_out: *mut u32) -> ZkbErr;
     pub fn zkb_program_free(prog: *mut ZkbProgram) -> ZkbErr;
     pub fn zkb_prover_set_program(p: *mut ZkbProver, prog: *mut ZkbProgram) -> ZkbErr;
+    pub fn zkb_session_new(h_circuit: *const u32, circuit_words: usize, devices: *const c_int, n_devices: usize, inflight: c_int, out: *mut *mut ZkbSession) -> ZkbErr;
+    pub fn zkb_session_commit(s: *mut ZkbSession, po2: c_int, h_code: *const c_void, h_control_id: *mut u32) -> ZkbErr;
+    pub fn zkb_session_control_ids(s: *mut ZkbSession, n: *mut usize, h_out: *mut u32) -> ZkbErr;
+    pub fn zkb_session_submit(s: *mut ZkbSession, po2: c_int, h_io: *const u32, h_data: *const c_void, h_accum: *const c_void, ticket: *mut u64) -> ZkbErr;
+    pub fn zkb_session_wait(s: *mut ZkbSession, ticket: u64, h_seal: *mut u32, words: *mut usize) -> ZkbErr;
+    pub fn zkb_session_free(s: *mut ZkbSession) -> ZkbErr;
     pub fn zkb_verify_segment(h_circuit: *const u32, circuit_words: usize, h_seal: *const u32, seal_words: usize, h_control_ids: *const u32, n_control_ids: usize, h_out_po2_code_root: *mut u32) -> ZkbErr;
     pub fn zkb_poseidon254_hash_rows(ctx: *mut ZkbCtx, d_out_digests: *mut c_void, d_matrix: *const c_void, rows: usize, cols: usize) -> ZkbErr;
     pub fn zkb_poseidon254_hash_fold(ctx: *mut ZkbCtx, d_nodes: *mut c_void, input_size: usize, output_size: usize) -> ZkbErr;

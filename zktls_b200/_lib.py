@@ -30,6 +30,7 @@ SYMBOLS = [
     "zkb_prover_seal_copy", "zkb_prover_root_count", "zkb_prover_roots_copy", "zkb_prove_segment", "zkb_prover_stage_traces",
     "zkb_prove_staged", "zkb_prover_stage_wait", "zkb_verify_segment",
     "zkb_program_new", "zkb_program_commit", "zkb_program_control_ids", "zkb_program_free", "zkb_prover_set_program",
+    "zkb_session_new", "zkb_session_commit", "zkb_session_control_ids", "zkb_session_submit", "zkb_session_wait", "zkb_session_free",
     "zkb_poseidon254_hash_rows", "zkb_poseidon254_hash_fold", "zkb_poseidon254_merkle_build", "zkb_poseidon254_permute_host",
 ]
 

@@ -4,9 +4,11 @@
 App. D.2): begin() commits `code` and `data` and returns the Fiat-Shamir `mix` globals the caller's accumulate step
 needs; finish() commits `accum` and finalizes; prove() is the one-shot form.  Traces may be numpy arrays (host) or
 `hal.Buffer`s (device).  `Program` commits a circuit's code trace once per po2 on a device; a prover that uses it takes
-code=None and proves from that commitment.
+code=None and proves from that commitment.  `Session` proves a queue of segments on every device from one object.
 """
 import ctypes as C
+import threading
+
 import numpy as np
 
 from ._lib import lib, check
@@ -57,6 +59,64 @@ class Program:
         """Releases this handle; provers that use the program keep it alive."""
         if self.h:
             check(lib().zkb_program_free(self.h)); self.h = C.c_void_p()
+
+
+class Session:
+    """The continuation segments of one session on one or more devices (zkb_session): `inflight` staged provers per device, one Program
+    per device, one queue.  commit() the code trace once per po2, submit() each segment's io and host traces (numpy arrays, ideally over
+    pinned memory) for a ticket, wait() for its seal.  submit and wait may be called from several threads.  devices=None: every visible
+    device."""
+
+    def __init__(self, circuit_blob, devices=None, inflight=3):
+        self.blob = np.ascontiguousarray(circuit_blob, dtype=np.uint32)
+        devs = None if devices is None else np.ascontiguousarray(devices, dtype=np.int32)
+        self.h = C.c_void_p()
+        self._keep, self._lock = {}, threading.Lock()      # ticket -> the traces the library reads until its seal is collected
+        check(lib().zkb_session_new(_hp(self.blob), _sz(self.blob.size), None if devs is None else devs.ctypes.data_as(C.POINTER(C.c_int)),
+                                    _sz(0 if devs is None else devs.size), C.c_int(inflight), C.byref(self.h)))
+
+    def commit(self, po2, code):
+        """Commits the host code trace at po2 on every device of the session; returns the control ID (po2, code root[8])."""
+        code = np.ascontiguousarray(code, dtype=np.uint32)
+        out = np.zeros(9, np.uint32)
+        check(lib().zkb_session_commit(self.h, C.c_int(po2), code.ctypes.data_as(C.c_void_p), _hp(out)))
+        return out
+
+    def control_ids(self):
+        """(k, 9) array of every committed (po2, code root), ascending po2: the table verify_segment takes."""
+        n = C.c_size_t(); check(lib().zkb_session_control_ids(self.h, C.byref(n), None))
+        out = np.zeros((n.value, 9), np.uint32)
+        check(lib().zkb_session_control_ids(self.h, C.byref(n), _hp(out)))
+        return out[: n.value]
+
+    def submit(self, po2, io, data, accum=None):
+        """Queues one segment and returns its ticket.  accum=None: the circuit's witness program computes the accum group on the device.
+        The arrays are kept alive until wait() or close()."""
+        io = np.ascontiguousarray(io, dtype=np.uint32)
+        arrs = [None if t is None else np.ascontiguousarray(t, dtype=np.uint32) for t in (data, accum)]
+        ptrs = [C.c_void_p(None) if a is None else a.ctypes.data_as(C.c_void_p) for a in arrs]
+        t = C.c_uint64()
+        with self._lock:          # the ticket is recorded before another thread can wait for it
+            check(lib().zkb_session_submit(self.h, C.c_int(po2), _hp(io), *ptrs, C.byref(t)))
+            self._keep[t.value] = arrs
+        return t.value
+
+    def wait(self, ticket):
+        """Blocks until the ticket's segment is proven; returns its seal, or raises the segment's own error.  Releases the ticket."""
+        try:
+            n = C.c_size_t(); check(lib().zkb_session_wait(self.h, C.c_uint64(ticket), None, C.byref(n)))
+            s = np.zeros(n.value, np.uint32)
+            check(lib().zkb_session_wait(self.h, C.c_uint64(ticket), _hp(s), C.byref(n)))
+            return s
+        finally:
+            with self._lock:
+                self._keep.pop(ticket, None)
+
+    def close(self):
+        """Fails the segments whose proof has not started, waits for the ones in progress, and frees the workers and programs."""
+        if self.h:
+            check(lib().zkb_session_free(self.h)); self.h = C.c_void_p()
+            self._keep.clear()
 
 
 class SegmentProver:

@@ -54,15 +54,17 @@ def trace_a(shape, po2, seed):
     return io, code, data, accum
 
 
-def trace_b_code_data(shape, po2, seed):
-    """Valid code + data columns (canonical values) and io.  Returns (io_mont, code_canon, data_canon)."""
+def trace_b_code_data(shape, po2, seed, code=None):
+    """Valid code + data columns (canonical values) and io.  Returns (io_mont, code_canon, data_canon).  code: a canonical code trace
+    of an earlier call to reuse (several segments of one program), else generated from the seed."""
     n = 1 << po2
     C, D = shape["code_cols"], shape["data_cols"]
     io = splitmix_fp(seed * 4 + 0, shape["out_size"])
-    code = splitmix_fp(seed * 4 + 1, C * n).reshape(C, n)
-    sel = np.zeros(n, dtype=np.uint64)
-    sel[1: n - ZK_ROWS] = 1
-    code[0] = sel
+    if code is None:
+        code = splitmix_fp(seed * 4 + 1, C * n).reshape(C, n)
+        sel = np.zeros(n, dtype=np.uint64)
+        sel[1: n - ZK_ROWS] = 1
+        code[0] = sel
     data = splitmix_fp(seed * 4 + 2, D * n).reshape(D, n)
     kidx = 1 + (np.arange(D) % (C - 1))
     for i in range(1, n - ZK_ROWS):
